@@ -55,7 +55,12 @@ def parse_args():
     ap.add_argument("--no-gather", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=20.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------
@@ -302,6 +307,29 @@ def cpu_reference_run(desc, args, inputs: np.ndarray, seconds: float):
                       % (n, cores, dt, t1)}
 
 
+DUMP_INSTANCES = 4          # instances of the batch written by --dump-outputs: the first, the last and two seeded ones
+DUMP_ENTRIES = 1 << 17      # witness entries per instance: a seeded sample when the witness is longer (4 x 2^17 x 64 B = 32 MB)
+
+
+def dump_outputs(out_dir: str, b, status: np.ndarray) -> None:
+    """What the timed path computed in its last step, as a caller receives it: the status of every instance
+    (status.npy) and the witness, as the .wtns holds it (canonical field elements), of a fixed, seeded sample of
+    instances (witness_instances.npy) and witness entries (witness_entries.npy).  witness.npy is
+    [instances][entries][8]: each 256-bit element as eight 32-bit limbs, least significant first, each exact in a float64.
+    The inputs are seeded, so two builds run with the same arguments can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    batch = status.shape[0]
+    rng = np.random.default_rng(7)
+    inst = np.unique(np.concatenate([[0, batch - 1], rng.integers(0, batch, DUMP_INSTANCES - 2)]))
+    rows = [np.frombuffer(b.wtns_bytes(int(i))[76:], dtype=np.uint32).reshape(-1, 8) for i in inst]   # 32-byte elements
+    n_wit = rows[0].shape[0]
+    ent = np.sort(rng.choice(n_wit, DUMP_ENTRIES, replace=False)) if n_wit > DUMP_ENTRIES else np.arange(n_wit)
+    arrays = {"status": status, "witness_instances": inst, "witness_entries": ent,
+              "witness": np.stack([r[ent] for r in rows])}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def native_lib():
     from circom_b200 import native
     return native.lib
@@ -341,7 +369,7 @@ class Ctx:
 
 def run_workload(ctx: Ctx, workload: str, batch: int, steps: int, warmup: int, e2e_steps: int, r1cs: bool,
                  parity_samples: int, lanes: int = 8, chain: int = 132, e2e_batch: int = 0, e2e_chunk: int = 0,
-                 sample_clocks: bool = False, gather: bool = False):
+                 sample_clocks: bool = False, gather: bool = False, dump_dir: str | None = None):
     """one workload on every rank; returns the result dict on every rank (only rank 0's is printed)"""
     import torch
     import torch.distributed as dist
@@ -388,6 +416,8 @@ def run_workload(ctx: Ctx, workload: str, batch: int, steps: int, warmup: int, e
     status = b.status()
     assert os.environ.get("CW_BENCH_NOCHECK") or not status.any(), "witness generation reported failing asserts: %r" % status[:8]
     bt_log2, threads, bytes_per_inst = b.layout()
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, b, status)
 
     # ---- parity: sampled witnesses of this run against the reference calculator -------------------
     parity = None
@@ -402,7 +432,7 @@ def run_workload(ctx: Ctx, workload: str, batch: int, steps: int, warmup: int, e
         r = R1cs(circuit)
         fb, _ = r.check_batch(b)
         assert (fb == -1).all(), "R1CS check failed on generated witnesses"
-        ms = [r.check_batch(b)[1] for _ in range(max(2, steps))]
+        ms = [r.check_batch(b)[1] for _ in range(steps)]
         r1cs_ms = ctx.max_over_ranks([float(np.mean(ms))])[0]
         try:   # which kernel decides the rows (integer rows: csrc/r1cs_small.h)
             r1cs_rows = r.compiled_info(b)
@@ -569,7 +599,8 @@ def main():
     _, _, batch = make_workload(args)
     out, desc, inputs = run_workload(ctx, args.workload, batch, args.steps, args.warmup, e2e_steps, not args.no_r1cs,
                                      parity_samples=2, lanes=args.lanes, chain=args.chain, e2e_batch=args.e2e_batch,
-                                     e2e_chunk=args.e2e_chunk, sample_clocks=True, gather=not args.no_gather)
+                                     e2e_chunk=args.e2e_chunk, sample_clocks=True, gather=not args.no_gather,
+                                     dump_dir=args.dump_outputs)
     if not args.no_configs and args.workload == "ecdsa_scale":
         # every BASELINE.json config at its stated per-GPU batch, each parity-gated against the reference calculator
         cfgs = []
@@ -577,7 +608,7 @@ def main():
                 ("C4", "sha256_512_bls", 1024, True, 4),
                 ("C3-calls: the headline circuit with its hints computed by circom-style functions", "ecdsa_scale_calls", 18944, False, 2)]
         for tag, wl, bsz, r1, ps in plan:
-            res, d2, in2 = run_workload(ctx, wl, bsz, max(3, min(args.steps, 5)), 3, 1, r1, parity_samples=ps,
+            res, d2, in2 = run_workload(ctx, wl, bsz, args.steps, 3, 1, r1, parity_samples=ps,
                                         lanes=args.lanes, chain=args.chain)
             res["config_id"] = tag
             if rank == 0 and world == 1 and not args.no_cpu_baseline and wl != args.workload:

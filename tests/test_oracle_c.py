@@ -1,11 +1,9 @@
 """The C oracle (oracle/cw_oracle.c) is pinned against the python model and against the REAL reference
 runtime: the reference's own main.cpp/calcwit.cpp/fr.cpp linked with the hand-lowered <circuit>.cpp
-(oracle/build_calcs.py) is run as `<bin> input.json out.wtns` and its bytes must equal the oracle's
-witness in .wtns framing (and, on the GPU box, the product's .wtns: tests/test_gpu_parity.py)."""
-import json
-import os
+(oracle/build_calcs.py), run as `<bin> input.json out.wtns`; the sha256 of the bytes it wrote and what it printed
+are stored in tests/golden/digests/reference.json, and the oracle's witness in .wtns framing must reproduce them
+(and, on a GPU, the product's .wtns: tests/test_gpu_parity.py)."""
 import random
-import subprocess
 
 import numpy as np
 import pytest
@@ -13,7 +11,7 @@ import pytest
 from oracle import build_calcs, c_oracle
 from oracle.field_model import Field, OPS
 from oracle.ir_eval import evaluate
-from tests.util import edge_values, flat_inputs, limbs_to_ints, rand_operand, PRIME_NAMES
+from tests.util import edge_values, flat_inputs, limbs_to_ints, rand_operand, reference_digests, sha256_hex, PRIME_NAMES
 from tests.test_lowering_cpu import CIRCUITS
 from circom_b200.circuit import CircuitDesc
 
@@ -74,12 +72,9 @@ REF_NAMES = ["multiplier2", "all_ops", "all_ops_bls", "less_than8", "poseidon2",
              "all_ops_gl", "less_than8_gl", "mixed_array_gl"]
 
 
-@pytest.mark.parametrize("name", REF_NAMES)
-def test_reference_runtime_wtns_equals_oracle(name, tmp_path):
-    calc = build_calcs.calc_path(name)
-    if not (os.path.exists(calc) and os.path.exists(calc + ".dat")):
-        pytest.skip("reference calculator %s not built (needs /root/reference; oracle/build_calcs.py)" % name)
-    d = build_calcs.make_desc(name)
+def runtime_inputs(d, name) -> np.ndarray:
+    """uint64 [2][n_in][4]: the inputs of the comparison (the reference calculator of the 1.2 M-constraint circuit ran on the
+    first only)"""
     rng = np.random.default_rng(11)
     n_in = d.main.n_in
     arr = np.zeros((2, n_in, 4), dtype=np.uint64)
@@ -103,23 +98,28 @@ def test_reference_runtime_wtns_equals_oracle(name, tmp_path):
         if d.prime == "goldilocks":   # values below q = 2^64 - 2^32 + 1
             arr[:, :, 1:] = 0
             arr[:, :, 0] &= np.uint64(0x7FFFFFFFFFFFFFFF)
+    return arr
+
+
+@pytest.mark.parametrize("name", REF_NAMES)
+def test_reference_runtime_wtns_equals_oracle(name):
+    ref = reference_digests()["runtime"][name]
+    d = build_calcs.make_desc(name)
+    arr = runtime_inputs(d, name)
+    assert len(ref) == (1 if "8x132" in name else 2)
     o = c_oracle.COracle(d.to_bytes())
     wit, st = o.run(arr)
     assert not st.any()
-    n_cases = 1 if "8x132" in name else 2
-    for i in range(n_cases):
-        jp, wp = str(tmp_path / "in.json"), str(tmp_path / "o.wtns")
-        json.dump(input_json(d, arr[i]), open(jp, "w"))
-        r = subprocess.run([calc, jp, wp], capture_output=True, text=True)
-        assert r.returncode == 0, r.stderr[-400:]
-        assert open(wp, "rb").read() == wtns_frame(d.q, wit[i])
+    for i, case in enumerate(ref):
+        assert sha256_hex(wtns_frame(d.q, wit[i])) == case["wtns_sha256"], (name, i)
         if d.strings:   # log() calls: what the calculator printed = cw_circuit_format_log of the witness, = the evaluator's text
             from circom_b200.witness_calculator import Circuit
             from oracle import ir_eval
+            stdout = case["stdout"]
             for o0 in (True, False):
                 c = Circuit(d, host_only=True, o0=o0)
                 w2s = c.witness2signal().astype(np.int64)
-                assert c.format_log(wit[i][w2s]) == r.stdout
+                assert c.format_log(wit[i][w2s]) == stdout
             ir_eval.LOG_SINK.clear()
             evaluate(d, {k: (int(v) if not isinstance(v, list) else [int(x) for x in v]) for k, v in input_json(d, arr[i]).items()})
-            assert "".join(ir_eval.LOG_SINK) == r.stdout and r.stdout.count("\n") == 4
+            assert "".join(ir_eval.LOG_SINK) == stdout and stdout.count("\n") == 4

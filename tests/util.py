@@ -2,6 +2,8 @@
 from __future__ import annotations
 
 import ctypes
+import hashlib
+import json
 import os
 import random
 import subprocess
@@ -120,3 +122,31 @@ def hostsim_run_r1cs(desc, inputs_list, flags=0, tamper=None):
                         fc.ctypes.data_as(ctypes.c_void_p), fp.ctypes.data_as(ctypes.c_void_p), cnt.ctypes.data_as(ctypes.c_void_p))
     assert rc == 0, (rc, hs.hs_last_error())
     return fc, fp, [int(x) for x in cnt]
+
+
+GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
+_digests = None
+
+
+def reference_digests() -> dict:
+    """What the reference's field library and witness calculators returned for the inputs the tests generate
+    (tests/golden/make_reference_digests.py): values, or the sha256 of long outputs."""
+    global _digests
+    if _digests is None:
+        with open(os.path.join(GOLDEN_DIR, "digests", "reference.json")) as f:
+            _digests = json.load(f)
+    return _digests
+
+
+def sha256_hex(raw: bytes) -> str:
+    return hashlib.sha256(raw).hexdigest()
+
+
+def digest_by_key(pairs, n8: int) -> dict:
+    """{key: [count, sha256 of the values, n8 bytes little-endian each, in order]} of (key, value) pairs"""
+    h = {}
+    for k, v in pairs:
+        e = h.setdefault(k, [0, hashlib.sha256()])
+        e[0] += 1
+        e[1].update(v.to_bytes(n8, "little"))
+    return {k: [n, s.hexdigest()] for k, (n, s) in sorted(h.items())}

@@ -286,8 +286,9 @@ static int get_dev_tape(const cw_circuit *c, int device, DevTape &out) {
 // fixed at compile time) / tile size as an argument
 template <int PR, bool CALLS, bool BP, int BT, bool FU>
 static void launch_tape_k(const TapeDev &tp, cw_batch *b, u32 tiles, u32 th) {
-    tape_exec_kernel<PR, CALLS, BP, BT, FU><<<tiles, th, 0, b->stream>>>(tp, b->slots, b->plane, b->bt_log2, b->first_assert_d,
-                                                                         b->err_d, b->batch);
+    static_assert(tape_acc_smem(CW_TAPE_LB) <= 48u * 1024u, "the accumulators of the widest CTA need an opt-in shared-memory size");
+    tape_exec_kernel<PR, CALLS, BP, BT, FU><<<tiles, th, FU ? tape_acc_smem(th) : 0u, b->stream>>>(
+        tp, b->slots, b->plane, b->bt_log2, b->first_assert_d, b->err_d, b->batch);
 }
 template <int PR>
 static void launch_tape(const TapeDev &tp, cw_batch *b, u32 tiles, u32 th, bool calls, bool bp, bool fused) {

@@ -116,7 +116,8 @@ struct Val {
 };
 
 // device-only opcodes (kernels.cuh / fr_device.cuh)
-enum { DOP_BITS = 29, DOP_ASSERT_BOOL = 30, DOP_MULSMALL = 31, DOP_BITSIP = 32, DOP_ASSERT_FITS = 33 };
+enum { DOP_BITS = 29, DOP_ASSERT_BOOL = 30, DOP_MULSMALL = 31, DOP_BITSIP = 32, DOP_ASSERT_FITS = 33,
+       DOP_ADD_NR = 34, DOP_ADD128 = 35, DOP_MULSMALL128 = 36, DOP_MULSMALL192 = 37, DOP_SHRI = 38, DOP_SHLI = 39 };
 inline bool c_is_immediate(uint32_t opcode) {
     return opcode == CW_OP_ASSERT || opcode == CW_OP_ASSERT_EQ || opcode == DOP_BITS || opcode == DOP_ASSERT_BOOL ||
            opcode == DOP_BITSIP || opcode == DOP_ASSERT_FITS;
@@ -1458,6 +1459,29 @@ struct Lowerer {
         for (const Val &v : vals)
             if (v.cid < 0 && v.slot[FC] != NO_SLOT && v.slot[FC] < slot_bits.size())
                 slot_bits[v.slot[FC]] = std::min<uint16_t>(slot_bits[v.slot[FC]], v.bits);
+        // ---- width-typed operators ------------------------------------------------------------------------------
+        // Where the range analysis proves an operator's canonical result narrow, the generic operator does work that
+        // cannot change the result: the modular correction of an addition below q, the limbs of an integer product
+        // above its width, the decoding of a constant shift amount (a 256-bit compare with q) and the reduction of a
+        // left shift below q.  Those operators become typed ones whose opcode says what is known (fr_device.cuh); the
+        // operands stay as they are.  Only the operators' own range analysis (Val::bits) is trusted here, not the
+        // widths of witness entries, which the circuit's constraints state but a failing instance may break.
+        if (!(flags & CW_FLAG_NO_TYPED)) {
+            const uint32_t lim = qb() - 1;
+            auto const_amount = [&](uint32_t o) {   // a constant operand below qbits
+                if (o == NO_SLOT || !(o & OPERAND_CONST)) return false;
+                const U256 &c = consts[o & ~OPERAND_CONST];
+                return !(c.v[1] | c.v[2] | c.v[3]) && c.v[0] < qb();
+            };
+            for (size_t i = 0; i < n_prov; ++i) {
+                uint32_t *o = &pops[i * 4];
+                const uint32_t bits = slot_bits[n_pre + i];
+                if (o[0] == CW_OP_ADD && bits <= lim) o[0] = bits <= 128 ? DOP_ADD128 : DOP_ADD_NR;
+                else if (o[0] == DOP_MULSMALL && bits <= 192) o[0] = bits <= 128 ? DOP_MULSMALL128 : DOP_MULSMALL192;
+                else if (o[0] == CW_OP_SHR && const_amount(o[2])) o[0] = DOP_SHRI;
+                else if (o[0] == CW_OP_SHL && bits <= lim && const_amount(o[2])) o[0] = DOP_SHLI;
+            }
+        }
         for (uint64_t i = 0; i < W; ++i) {  // copies made for the witness carry their entry's width
             uint32_t wb = vbits(sig_vid[T.witness2signal[i]]);
             slot_bits[wsrc[i]] = std::min<uint16_t>(slot_bits[wsrc[i]], (uint16_t)wb);
@@ -2002,7 +2026,7 @@ struct BlobR {
         p += n;
     }
 };
-constexpr uint32_t BLOB_VERSION = 6;
+constexpr uint32_t BLOB_VERSION = 7;
 }  // namespace
 
 void serialize_tape(const Tape &t, std::vector<uint8_t> &out) {

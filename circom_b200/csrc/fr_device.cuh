@@ -638,7 +638,8 @@ CW_HD bool u256_divmod(u32 *quo, u32 *rem, const u32 *a, const u32 *b) {
 
 // ---- one tape instruction ----------------------------------------------------------------------
 // Opcodes are cw_op (include/circom_b200.h).  Operands arrive in the representation the lowering
-// chose (flatten.cpp); `err` is set to 1 on division by zero.  Returns true if r holds a result.
+// chose (flatten.cpp); `err` is set to 1 on division by zero (host builds: also on a typed operator whose range
+// claim fails, below).  Returns true if r holds a result.
 enum {
     OP_MUL = 1, OP_ADD = 3, OP_SUB = 4, OP_POW = 5, OP_IDIV = 6, OP_MOD = 7, OP_SHL = 8, OP_SHR = 9,
     OP_LEQ = 10, OP_GEQ = 11, OP_LT = 12, OP_GT = 13, OP_EQ = 14, OP_NEQ = 15, OP_LOR = 16, OP_LAND = 17,
@@ -648,7 +649,16 @@ enum {
     OP_ASSERT_BOOL = 30,  // a == 0 || a == b  (b = the constant one in a's representation)
     OP_MULSMALL = 31,     // a * b as integers, statically known to stay below q (no reduction)
     OP_BITSIP = 32,       // a & ((2^len - 1) << lo), imm = lo | len << 8  (sum of adjacent bit fields)
-    OP_ASSERT_FITS = 33   // a < 2^m, m = b[0]  (recomposition check of a bit decomposition)
+    OP_ASSERT_FITS = 33,  // a < 2^m, m = b[0]  (recomposition check of a bit decomposition)
+    // width-typed operators: the lowering's range analysis proves the canonical result narrow, so the integer result
+    // is the field result and only the limbs that can be non-zero are computed.  (Below FOP_JMP: OP_CALL must stay the
+    // largest opcode of a level.)
+    OP_ADD_NR = 34,        // a + b < q: no modular correction
+    OP_ADD128 = 35,        // a + b < 2^128: a 4-limb addition
+    OP_MULSMALL128 = 36,   // a * b < 2^128 as integers: the low 4 limbs of the product
+    OP_MULSMALL192 = 37,   // a * b < 2^192 as integers: the low 6 limbs
+    OP_SHRI = 38,          // a >> b, b a constant below qbits (no decoding of the amount against q)
+    OP_SHLI = 39           // a << b, b a constant below qbits, the result proved below q (no reduction)
 };
 
 // low 256 bits of the integer product (36 limb products instead of CIOS' 128)
@@ -667,6 +677,35 @@ CW_HD void u256_mul_lo(u32 *r, const u32 *a, const u32 *b) {
         }
     }
     u256_set(r, t);
+}
+// low K limbs of the integer product, the limbs above them zero (K (K + 1) / 2 limb products)
+template <int K>
+CW_HD void u256_mul_lo_k(u32 *r, const u32 *a, const u32 *b) {
+    u32 t[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) t[i] = 0;
+#pragma unroll
+    for (int i = 0; i < K; ++i) {
+        u64 c = 0;
+#pragma unroll
+        for (int j = 0; j + i < K; ++j) {
+            c += (u64)a[j] * b[i] + t[i + j];
+            t[i + j] = (u32)c;
+            c >>= 32;
+        }
+    }
+    u256_set(r, t);
+}
+CW_HD void u256_add_lo4(u32 *r, const u32 *a, const u32 *b) {   // a + b < 2^128
+    u64 c = 0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        c += (u64)a[i] + b[i];
+        r[i] = (u32)c;
+        c >>= 32;
+    }
+#pragma unroll
+    for (int i = 4; i < 8; ++i) r[i] = 0;
 }
 CW_HD void u256_bits(u32 *r, const u32 *a, u32 imm) {
     u32 k = imm & 0xFFFFu, m = (imm >> 16) & 0xFFu;
@@ -707,6 +746,16 @@ CW_HD u32 u256_bitlen(const u32 *a) {
     return n;
 }
 
+// a width-typed operator's result r equals the generic operator's, and is below q
+CW_HD bool fr_typed_holds(u32 opcode, const u32 *r, const u32 *a, const u32 *b, const FrParams &P) {
+    u32 g[8];
+    if (opcode == OP_ADD_NR || opcode == OP_ADD128) fr_add(g, a, b, P);
+    else if (opcode == OP_MULSMALL128 || opcode == OP_MULSMALL192) u256_mul_lo(g, a, b);
+    else if (opcode == OP_SHRI) fr_shr(g, a, b, P);
+    else fr_shl(g, a, b, P);
+    return u256_eq(g, r) && !u256_geq(r, P.q);
+}
+
 // SLOW = false leaves out the two operators that are loops of hundreds of steps (INV, POW): the interpreter runs them
 // in a pass of their own so that their code and registers stay out of its hot loop (kernels.cuh)
 template <bool SLOW>
@@ -715,8 +764,14 @@ CW_HD void fr_exec_t(u32 opcode, u32 *r, const u32 *a, const u32 *b, u32 imm, co
         case OP_BITSIP: u256_bits_in_place(r, a, imm); break;
         case OP_BITS: u256_bits(r, a, imm); break;
         case OP_MULSMALL: u256_mul_lo(r, a, b); break;
+        case OP_MULSMALL128: u256_mul_lo_k<4>(r, a, b); break;
+        case OP_MULSMALL192: u256_mul_lo_k<6>(r, a, b); break;
         case OP_MUL: fr_mont_mul(r, a, b, P); break;
         case OP_ADD: fr_add(r, a, b, P); break;
+        case OP_ADD_NR: u256_add(r, a, b); break;
+        case OP_ADD128: u256_add_lo4(r, a, b); break;
+        case OP_SHRI: u256_shr(r, a, b[0]); break;
+        case OP_SHLI: u256_shl(r, a, b[0]); break;
         case OP_SUB: fr_sub(r, a, b, P); break;
         case OP_NEG: fr_neg(r, a, P); break;
         case OP_INV: if (SLOW) fr_inv_mont(r, a, P); break;
@@ -757,6 +812,11 @@ CW_HD void fr_exec_t(u32 opcode, u32 *r, const u32 *a, const u32 *b, u32 imm, co
         case OP_COPY: u256_set(r, a); break;
         default: u256_set_u32(r, 0); break;
     }
+#if !defined(__CUDA_ARCH__)
+    // host builds (the simulator the CPU tests run tapes on): a typed operator also checks the claim of the range
+    // analysis it rests on; a violation is reported like a division by zero, as an error of the instance
+    if (opcode >= OP_ADD_NR && opcode <= OP_SHLI && !fr_typed_holds(opcode, r, a, b, P)) err = 1;
+#endif
 }
 CW_HD void fr_exec(u32 opcode, u32 *r, const u32 *a, const u32 *b, u32 imm, const FrParams &P, int &err) {
     fr_exec_t<true>(opcode, r, a, b, imm, P, err);

@@ -213,6 +213,22 @@ __device__ __noinline__ void exec_call(const TapeDev &tp, u32 call_off, uint4 *b
     *err = e;
 }
 
+// ---- the accumulators of fused work items ----------------------------------------------------------------
+// A fused work item keeps the values its inner words produce in two accumulators.  They live in shared memory, not
+// in registers: 16 registers of accumulators, plus the selects between them that a register array indexed by a tape
+// bit needs, pushed the fused interpreter over its 64-register budget into local-memory spills around every word.
+// Layout [acc][half][thread] (uint4): a warp moves one 512-byte row per half, without bank conflicts.
+__host__ __device__ constexpr unsigned tape_acc_smem(unsigned threads) { return 4u * threads * (unsigned)sizeof(uint4); }
+__device__ __forceinline__ void load_acc(u32 *v, const uint4 *s_acc, u32 k) {
+    const uint4 lo = s_acc[(2u * k) * blockDim.x + threadIdx.x], hi = s_acc[(2u * k + 1u) * blockDim.x + threadIdx.x];
+    v[0] = lo.x; v[1] = lo.y; v[2] = lo.z; v[3] = lo.w;
+    v[4] = hi.x; v[5] = hi.y; v[6] = hi.z; v[7] = hi.w;
+}
+__device__ __forceinline__ void store_acc(const u32 *v, uint4 *s_acc, u32 k) {
+    s_acc[(2u * k) * blockDim.x + threadIdx.x] = make_uint4(v[0], v[1], v[2], v[3]);
+    s_acc[(2u * k + 1u) * blockDim.x + threadIdx.x] = make_uint4(v[4], v[5], v[6], v[7]);
+}
+
 // HAS_CALLS selects the build that contains the function interpreter (more registers, a local-memory
 // frame); tapes without calls - all circuits whose hints are straight-line - use the lean build.
 // BP: the tape was lowered with a bit plane (bit runs write plane words, operands may be plane bits).
@@ -220,7 +236,7 @@ __device__ __noinline__ void exec_call(const TapeDev &tp, u32 call_off, uint4 *b
 #define CW_TAPE_LB 512  // widest CTA of the interpreter (cw_batch_create clamps to it); with MINB it bounds the registers
 #endif
 #ifndef CW_TAPE_MINB
-#define CW_TAPE_MINB 2  // 512 x 2: a 64-register budget (the fused build spills ~100 bytes; measured faster than 84 registers)
+#define CW_TAPE_MINB 2  // 512 x 2: a 64-register budget (measured faster than 84 registers)
 #endif
 // BT >= 0 fixes the tile size at compile time (BT = 0, one instance per CTA: the slot address arithmetic then
 // folds to `base + slot * 32`; BT = 5, a warp per op); BT < 0 takes it from the launch argument.
@@ -237,6 +253,8 @@ __global__ void __launch_bounds__(CW_TAPE_LB, CW_TAPE_MINB)
     const u32 bt_mask = (1u << bt_log2) - 1;
     uint4 *base = slots + (((size_t)tile * tp.n_slots) << (bt_log2 + 1));
     u32 *plane_base = BP ? plane + (((size_t)tile * tp.n_bitwords) << bt_log2) : nullptr;
+    // FUSED: the two accumulators of the thread's work item (tape_acc_smem bytes of dynamic shared memory)
+    extern __shared__ uint4 s_acc[];
     u32 lb = tp.level_start[0];
     u32 le = tp.n_levels ? tp.level_start[1] : lb;
     // the first tape word of a thread's first work item of the next level is fetched before the barrier of the
@@ -272,9 +290,6 @@ __global__ void __launch_bounds__(CW_TAPE_LB, CW_TAPE_MINB)
                 g0 = first ? pre_g0 : __ldg(&tp.items[lb + (w >> bt_log2)]);
                 g1 = first ? pre_g1 : __ldg(&tp.items[lb + (w >> bt_log2) + 1]);
             }
-            // a fused work item: its words run back to back in this thread, single-use values stay in two
-            // accumulator registers instead of travelling through the value store
-            u32 acc0[8], acc1[8];
             uint4 nxt = pre;
             if (!first) {
                 if (FUSED) nxt = __ldg(&tp.heads[lb + (w >> bt_log2)]);
@@ -321,14 +336,10 @@ __global__ void __launch_bounds__(CW_TAPE_LB, CW_TAPE_MINB)
                 } else r[0] = (u32)window & (m >= 32u ? 0xFFFFFFFFu : ((1u << m) - 1u));
             } else {
                 u32 a[8], b[8];
-                if (FUSED && !(opw.y & OPD_CONST) && (opw.y & OPD_ACC)) {
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) a[i] = (opw.y & 1u) ? acc1[i] : acc0[i];
-                } else load_operand<BP>(a, opw.y, base, plane_base, tp.consts, bt_log2, li);
-                if (FUSED && !(opw.z & OPD_CONST) && (opw.z & OPD_ACC)) {
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) b[i] = (opw.z & 1u) ? acc1[i] : acc0[i];
-                } else load_operand<BP>(b, opw.z, base, plane_base, tp.consts, bt_log2, li);
+                if (FUSED && !(opw.y & OPD_CONST) && (opw.y & OPD_ACC)) load_acc(a, s_acc, opw.y & 1u);
+                else load_operand<BP>(a, opw.y, base, plane_base, tp.consts, bt_log2, li);
+                if (FUSED && !(opw.z & OPD_CONST) && (opw.z & OPD_ACC)) load_acc(b, s_acc, opw.z & 1u);
+                else load_operand<BP>(b, opw.z, base, plane_base, tp.consts, bt_log2, li);
                 if (opcode == OP_SELECT) {
                     u32 c[8];
                     load_operand<BP>(c, opw.w, base, plane_base, tp.consts, bt_log2, li);
@@ -352,13 +363,8 @@ __global__ void __launch_bounds__(CW_TAPE_LB, CW_TAPE_MINB)
                 }
             }
             if (has_value) {
-                if (FUSED && dst >= DST_ACC_DEV) {
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        if (dst & 1u) acc1[i] = r[i];
-                        else acc0[i] = r[i];
-                    }
-                } else store_slot(r, base, dst, bt_log2, li);
+                if (FUSED && dst >= DST_ACC_DEV) store_acc(r, s_acc, dst & 1u);
+                else store_slot(r, base, dst, bt_log2, li);
             }
             }
             }

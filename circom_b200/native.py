@@ -15,6 +15,7 @@ CW_OK, CW_EINVAL, CW_EIO, CW_EFORMAT, CW_ECUDA, CW_ENOTFOUND, CW_ESTATE, CW_ENOD
 CW_FLAG_NO_ASSERTS, CW_FLAG_HOST_ONLY, CW_FLAG_O0, CW_FLAG_NO_PEEPHOLE, CW_FLAG_BITPLANE, CW_FLAG_REUSE = 1, 2, 4, 8, 16, 32
 CW_FLAG_COMPACT = CW_FLAG_BITPLANE | CW_FLAG_REUSE
 CW_FLAG_FUSE = 64
+CW_FLAG_NO_TYPED = 128
 
 
 class CwError(RuntimeError):

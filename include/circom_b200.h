@@ -54,9 +54,11 @@ extern "C" {
 #define CW_FLAG_NO_PEEPHOLE 8u /* lower IR ops one to one (no bit-field / boolean-assert / shift fusions) */
 #define CW_FLAG_BITPLANE 16u   /* bits written by bit runs live in a packed per-instance bit plane */
 #define CW_FLAG_REUSE 32u      /* values that are not witness entries share slots (allocated like registers) */
-#define CW_FLAG_FUSE 64u       /* single-use values are evaluated inside their reader's work item (two accumulator registers) instead
+#define CW_FLAG_FUSE 64u       /* single-use values are evaluated inside their reader's work item (two accumulators) instead
                                   of travelling through the value store: half the levels, 30 % fewer stores; pays only for large
                                   batches (measured: DESIGN.md section 7) */
+#define CW_FLAG_NO_TYPED 128u /* keep the generic operators where the range analysis proves a narrower one exact (width-typed
+                                  additions, multiplications and constant shifts; for A/B measurements and parity tests) */
 #define CW_FLAG_COMPACT (CW_FLAG_BITPLANE | CW_FLAG_REUSE) /* the compact value store: what cw_batch_* runs best on */
 #define CW_FLAG_O0 4u         /* --O0: keep every signal in the witness and every `signal = signal` constraint */
 
